@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - PCG iterations/s and SpMV GB/s (fp64) on B200, next to the CPU reference path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--block 128]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--block 128] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1] at N=1, the C5 stacking rule at N>1, weak scaling): every GPU owns
@@ -286,6 +286,28 @@ def preflight_parity(comm, dev, rank, world, block=6):
     return res
 
 
+# --------------------------------------------------------------------------------------- outputs
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def dump_outputs(path, x, info, rank, world):
+    """Writes the timed solve's outputs: x (float64, this rank's subdomain) as x.npy, or x_rank<r>.npy when N > 1, and
+    solve_info.npy = [flag, iterations, relres] (float64, the same on every rank).  The files of all ranks stay within
+    DUMP_BUDGET_BYTES: a rank whose x does not fit its share writes a fixed sample of it instead (seed 0, ascending dof
+    indices, the same for every run of the same mesh) and those indices as <name>_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    name = "x" if world == 1 else f"x_rank{rank}"
+    xh = x.detach().cpu().numpy().astype(np.float64, copy=False)
+    keep = (DUMP_BUDGET_BYTES - 4096) // world // 8
+    if xh.size > keep:
+        idx = np.sort(np.random.default_rng(0).choice(xh.size, keep // 2, replace=False))   # half for values, half for indices
+        xh = xh[idx]
+        np.save(os.path.join(path, f"{name}_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, f"{name}.npy"), xh)
+    if rank == 0:
+        np.save(os.path.join(path, "solve_info.npy"), np.array([info.flag, info.iters, info.relres], dtype=np.float64))
+
+
 # --------------------------------------------------------------------------------------- main
 def main():
     import faulthandler
@@ -305,7 +327,12 @@ def main():
     ap.add_argument("--operator", default="csr", choices=["csr", "ebe"],
                     help="csr = assembled merge-path SpMV (the north-star path, default); ebe = opt-in matrix-free operator (f1)")
     ap.add_argument("--e2e-repeats", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed solve returned (its solution x and flag / iterations / "
+                         "relative residual) to DIR as .npy files, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -505,6 +532,10 @@ def main():
         full_solve = {"tol": 1e-8, "flag": fi.flag, "iterations": fi.iters, "relres": fi.relres, "loop_ms": max_over_ranks(fi.loop_ms),
                       "iterations_per_s": fi.iters / (max_over_ranks(fi.loop_ms) * 1e-3), "time_to_solution_s": max_over_ranks(wall),
                       "reference_published_s": 12.6, "reference_published_note": "notebooks/solver_demo.ipynb:380-408: tol 1e-7, 1085 iterations, 8 cores"}
+        barrier()
+
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, info, rank, world)
         barrier()
 
     rc = 0

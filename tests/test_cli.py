@@ -10,24 +10,19 @@ import pytest
 
 from oracle import ref_pcg as R
 from oracle import run_reference as rr
-from oracle.hex_mdf import write_hex_mdf
+from oracle.cli_workdir import FRAME_CASES, same_fixture, setup_workdir
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-def _setup_workdir(tmp_path, ng, tol, maxiter, deltas=(0, 1)):
-    """A work directory laid out like read_input_model.py leaves it (read_input_model.py:24-48)."""
-    from pcg_mpi_solver_b200.pcg_solver import exportz
-    work = str(tmp_path)
-    mdf = os.path.join(work, "data", "ModelData", "MDF") + "/"
-    info = write_hex_mdf(mdf, ng)
-    os.makedirs(os.path.join(work, "__pycache__"), exist_ok=True)
-    os.makedirs(os.path.join(work, "data", "ModelData", "MPI"), exist_ok=True)   # read_input_model.py:31-36
-    exportz(os.path.join(work, "__pycache__", "ModelDataPaths.zpkl"),
-            {"ScratchPath": os.path.join(work, "data"), "MDF_Path": mdf, "PyDataPath_Part": os.path.join(work, "data", "ModelData", "MPI") + "/",
-             "ModelName": "hexmodel"})
-    rr.write_settings(work, tol, maxiter, deltas)
-    return work, mdf, info
+def _unpack_reference_files(prefix, dst):
+    """Writes the files that the unmodified reference produced under `prefix` of tests/golden/cli_ref.npz
+    (oracle/make_golden_cli.py) into the directory `dst`."""
+    os.makedirs(dst, exist_ok=True)
+    with np.load(os.path.join(GOLD, "cli_ref.npz")) as z:
+        for key in z.files:
+            if key.startswith(prefix + "/") and "/" not in key[len(prefix) + 1:]:
+                z[key].tofile(os.path.join(dst, key[len(prefix) + 1:]))
 
 
 def _oracle_backend(mp, ranks):
@@ -60,7 +55,7 @@ def test_cli_file_formats_roundtrip_cpu(tmp_path):
         meta = json.load(f)
     gold = np.load(os.path.join(GOLD, "hex_ref.npz"))
     ng = tuple(meta["ng"])
-    work, mdf, info = _setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
+    work, mdf, info = setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
     subs = partition_mesh(load_mdf(mdf, "hexmodel"), 1, assemble=False)
     prefix = os.path.join(work, "data", "ModelData", "MPI") + "/"
     export_mesh_parts(prefix, subs)
@@ -84,7 +79,7 @@ def test_cli_multi_step_ramp_cpu(tmp_path):
     from pcg_mpi_solver_b200.model import load_mdf
     from pcg_mpi_solver_b200.partition import partition_mesh
     from pcg_mpi_solver_b200.pcg_solver import export_mesh_parts, run
-    work, mdf, info = _setup_workdir(tmp_path, (4, 3, 3), 1e-11, 2000, deltas=(0, 0.5, 1.0))
+    work, mdf, info = setup_workdir(tmp_path, (4, 3, 3), 1e-11, 2000, deltas=(0, 0.5, 1.0))
     subs = partition_mesh(load_mdf(mdf, "hexmodel"), 1, assemble=False)
     export_mesh_parts(os.path.join(work, "data", "ModelData", "MPI") + "/", subs)
     out = run(7, 0, workdir=work, backend=_oracle_backend, quiet=True)
@@ -94,13 +89,12 @@ def test_cli_multi_step_ramp_cpu(tmp_path):
     assert np.linalg.norm(u2 - 2.0 * u1) <= 1e-8 * np.linalg.norm(u2)   # linear problem: delta 1.0 vs 0.5
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/solver/partition_mesh.py"), reason="needs the reference checkout")
 def test_cli_reads_the_reference_builders_fixture_cpu(tmp_path):
     """The fixture written by the UNMODIFIED reference builder is consumed as is."""
     from pcg_mpi_solver_b200.pcg_solver import run
-    work, mdf, info = _setup_workdir(tmp_path, (5, 4, 3), 1e-10, 3000)
-    rr.metis_stage(work, 1)
-    rr.partition_stage(work, 1)                       # reference's partition_mesh.py under the shim -> 1_0.mpidat
+    work, mdf, info = setup_workdir(tmp_path, (5, 4, 3), 1e-10, 3000)
+    # the reference's run_metis.py + partition_mesh.py on this model -> 1_metadat.npy, 1_0.mpidat
+    _unpack_reference_files("fixture_543", os.path.join(work, "data", "ModelData", "MPI"))
     out = run(3, 0, workdir=work, backend=_oracle_backend, quiet=True)
     assert out["Flag"][1] == 0
     A = R.hex_box_csr((5, 4, 3), (0, 0, 0), (5, 4, 3), h=info["h"])
@@ -109,23 +103,21 @@ def test_cli_reads_the_reference_builders_fixture_cpu(tmp_path):
     assert np.linalg.norm(b - A @ x) <= 1e-10 * np.linalg.norm(b) * (1 + 1e-6)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/solver/pcg_solver.py"), reason="needs the reference checkout")
-@pytest.mark.parametrize("rate,frms", [(0, [[2, 3]]), (2, [[2]]), (0, [])])
+@pytest.mark.parametrize("rate,frms", FRAME_CASES)
 def test_cli_export_frames_match_the_reference(tmp_path, rate, frms):
     """ExportFrms is a NESTED, 1-BASED list (np.array(ExportFrms, int)[0] - 1, pcg_solver.py:156-159) and the step-0 frame is
     written only when the ExportNow predicate holds for step 0 (:854-859): same set of U_k files, same contents, same Time_T
-    as the unmodified reference run on the same fixture."""
+    as the unmodified reference run on the same fixture (its result files: tests/golden/cli_ref.npz)."""
     from pcg_mpi_solver_b200.pcg_solver import run
-    work, mdf, info = _setup_workdir(tmp_path, (4, 3, 3), 1e-11, 2000)
-    rr.metis_stage(work, 1)
-    rr.partition_stage(work, 1)
+    work, mdf, info = setup_workdir(tmp_path, (4, 3, 3), 1e-11, 2000)
+    _unpack_reference_files("fixture_433", os.path.join(work, "data", "ModelData", "MPI"))
     settings = {"TimeHistoryParam": {"ExportFlag": True, "ExportFrmRate": rate, "ExportFrms": frms, "PlotFlag": False,
                                      "TimeStepDelta": [0, 0.25, 0.5, 1.0], "ExportVars": "U"}, "SolverParam": {"Tol": 1e-11, "MaxIter": 2000}}
     with open(os.path.join(work, "__pycache__", "GlobSettings.zpkl"), "wb") as f:
         f.write(zlib.compress(pickle.dumps(settings, pickle.HIGHEST_PROTOCOL)))
-    rr.solve_stage(work, 1, run_id=1)                                    # the unmodified reference
+    ref_dir = os.path.join(work, "reference_ResVecData")                 # the unmodified reference's run on this fixture
+    _unpack_reference_files(f"frames{FRAME_CASES.index((rate, frms))}", ref_dir)
     run(2, 0, workdir=work, backend=_oracle_backend, quiet=True)         # the file-compatible stage
-    ref_dir = os.path.join(work, "data", "Results_Run1", "ResVecData")
     our_dir = os.path.join(work, "data", "Results_Run2", "ResVecData")
     ref_files = sorted(f for f in os.listdir(ref_dir) if f.endswith(".mpidat"))
     assert sorted(f for f in os.listdir(our_dir) if f.endswith(".mpidat")) == ref_files
@@ -152,7 +144,7 @@ def test_cli_on_gpu_matches_reference_golden(cuda, tmp_path):
         meta = json.load(f)
     gold = np.load(os.path.join(GOLD, "hex_ref.npz"))
     ng = tuple(meta["ng"])
-    work, mdf, info = _setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
+    work, mdf, info = setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
     subs = partition_mesh(load_mdf(mdf, "hexmodel"), 1, assemble=False)
     export_mesh_parts(os.path.join(work, "data", "ModelData", "MPI") + "/", subs)
     run(1, 0, workdir=work, quiet=True)
@@ -162,26 +154,32 @@ def test_cli_on_gpu_matches_reference_golden(cuda, tmp_path):
     assert np.linalg.norm(u - gold["U_box1"]) <= 1e-8 * np.linalg.norm(gold["U_box1"])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/solver/pcg_solver.py"), reason="needs the reference checkout")
 @pytest.mark.parametrize("nparts", [1, 2])
 def test_reference_solver_consumes_the_product_builders_fixture(tmp_path, nparts):
-    """Drop-in the other way round: the UNMODIFIED reference solver (pcg_solver.py under the fake-MPI shim) runs on the
-    fixture written by the product's partition_mesh()/export_mesh_parts() and reproduces its own golden run."""
-    from pcg_mpi_solver_b200.hexmesh import block_grid, partition_blocks
+    """Drop-in the other way round: the UNMODIFIED reference solver (pcg_solver.py under the fake-MPI shim) ran on the
+    fixture written by the product's partition_mesh()/export_mesh_parts() and reproduced its own golden run
+    (oracle/make_golden_cli.py stored that fixture and the reference's result): the builder still writes that fixture."""
     from pcg_mpi_solver_b200.model import load_mdf
     from pcg_mpi_solver_b200.partition import partition_mesh
-    from pcg_mpi_solver_b200.pcg_solver import export_mesh_parts
+    from pcg_mpi_solver_b200.pcg_solver import export_mesh_parts, read_mesh_part
     with open(os.path.join(GOLD, "hex_ref.json")) as f:
         meta = json.load(f)
     gold = np.load(os.path.join(GOLD, "hex_ref.npz"))
     ng = tuple(meta["ng"])
-    work, mdf, info = _setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
+    work, mdf, info = setup_workdir(tmp_path, ng, meta["tol"], meta["maxiter"])
     case = "box1" if nparts == 1 else "box2"
     ep = gold[f"elepart_{case}"].astype(np.int64) if nparts > 1 else None
     subs = partition_mesh(load_mdf(mdf, "hexmodel"), nparts, elepart=ep, assemble=False)
-    export_mesh_parts(os.path.join(work, "data", "ModelData", "MPI") + "/", subs)
-    rr.solve_stage(work, nparts, run_id=5)                      # /root/reference/src/solver/pcg_solver.py, one process per part
-    res, u = rr.read_results(work, "hexmodel", nparts, 5, info["ndof"])
+    prefix = os.path.join(work, "data", "ModelData", "MPI") + "/"
+    export_mesh_parts(prefix, subs)
+    ref_prefix = os.path.join(work, "consumed_by_reference") + "/"
+    _unpack_reference_files(f"consumes{nparts}/fixture", ref_prefix)
+    for p in range(nparts):
+        assert same_fixture(read_mesh_part(prefix, nparts, p), read_mesh_part(ref_prefix, nparts, p)), p
+    # the reference's run (pcg_solver.py, one process per part) on that fixture, as recorded: these asserts compare two
+    # golden files (cli_ref.npz and hex_ref.npz) and compute nothing; they keep a regenerated cli_ref.npz honest
+    with np.load(os.path.join(GOLD, "cli_ref.npz")) as z:
+        flag, iters, u = int(z[f"consumes{nparts}/Flag"]), int(z[f"consumes{nparts}/Iter"]), z[f"consumes{nparts}/U"]
     run = meta["runs"][case]
-    assert res["Flag"] == 0 and res["Iter"] == run["Iter"]
+    assert flag == 0 and iters == run["Iter"]
     assert np.linalg.norm(u - gold[f"U_{case}"]) <= 1e-12 * np.linalg.norm(gold[f"U_{case}"])

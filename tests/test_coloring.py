@@ -37,8 +37,6 @@ def test_concrete_colouring():
     from pcg_mpi_solver_b200.model import load_mdf
     zp = os.path.join(ROOT, "oracle", "_ref", "concrete.zip")
     if not os.path.exists(zp):
-        zp = "/root/reference/data/concrete.zip"
-    if not os.path.exists(zp):
         pytest.skip("concrete.zip not staged")
     m = load_mdf(zp)
     ptr = np.concatenate([m.node_offset[:, 0], m.node_offset[-1:, 1] + 1])

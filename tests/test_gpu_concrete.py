@@ -12,10 +12,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _zip():
-    for p in (os.path.join(ROOT, "oracle", "_ref", "concrete.zip"), "/root/reference/data/concrete.zip"):
-        if os.path.exists(p):
-            return p
-    pytest.skip("data/concrete.zip not staged")
+    p = os.path.join(ROOT, "oracle", "_ref", "concrete.zip")
+    if not os.path.exists(p):
+        pytest.skip("data/concrete.zip not staged")
+    return p
 
 
 @pytest.fixture(scope="module")

@@ -21,10 +21,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _concrete_zip():
-    for p in (os.path.join(ROOT, "oracle", "_ref", "concrete.zip"), "/root/reference/data/concrete.zip"):
-        if os.path.exists(p):
-            return p
-    pytest.skip("data/concrete.zip not staged (run __graft_entry__.build() where /root/reference exists)")
+    p = os.path.join(ROOT, "oracle", "_ref", "concrete.zip")
+    if not os.path.exists(p):
+        pytest.skip("data/concrete.zip not staged (__graft_entry__.build() stages it where the reference checkout is readable)")
+    return p
 
 
 @pytest.fixture(scope="module")
