@@ -28,6 +28,7 @@ import torch
 
 from . import _lib
 from .csr import CsrMatrix
+from .ebe import EbeMatrix
 
 
 def _allgather_bytes(blob: bytes, group=None):
@@ -164,6 +165,10 @@ class SubdomainOperator:
 
     def __init__(self, A, comm: Communicator | None = None, nbr_ranks=(), ovrlp=(), weights=None,
                  n_global: int | None = None):
+        # the C side reads A.handle as a pcgb_csr_t or a pcgb_ebe_t: any other handle (EbeMatrixColored holds a
+        # pcgb_ebe2_t) would be misread as one of them, so it is refused before anything reaches the library
+        if not isinstance(A, (CsrMatrix, EbeMatrix)):
+            raise TypeError(f"SubdomainOperator: A must be a CsrMatrix or an EbeMatrix, not {type(A).__name__}")
         self.A, self.comm = A, comm
         self.n = A.shape[0]
         self.device = A.device

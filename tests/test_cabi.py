@@ -37,6 +37,25 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_lib.EbeGroup) == sizes[3]
 
 
+def test_operator_refuses_foreign_matrix_handles(monkeypatch):
+    """SubdomainOperator hands A.handle to the library as a pcgb_csr_t or a pcgb_ebe_t.  Anything else - an
+    EbeMatrixColored holds a pcgb_ebe2_t - is refused with TypeError before any call into the library."""
+    import torch
+    from pcg_mpi_solver_b200 import _lib
+    from pcg_mpi_solver_b200.ebe import EbeMatrixColored
+    from pcg_mpi_solver_b200.solver import SubdomainOperator
+
+    def no_library(*args, **kwargs):
+        raise AssertionError("the library was called")
+
+    monkeypatch.setattr(_lib, "load", no_library)
+    colored = EbeMatrixColored.__new__(EbeMatrixColored)    # a handle-carrying object of the wrong kind, no device needed
+    colored.shape, colored.device, colored._h = (6, 6), torch.device("cpu"), ctypes.c_void_p()
+    for A in (colored, object()):
+        with pytest.raises(TypeError, match="CsrMatrix or an EbeMatrix"):
+            SubdomainOperator(A)
+
+
 def test_no_cpu_fallback():
     import numpy as np
     import torch

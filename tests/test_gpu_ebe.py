@@ -28,6 +28,9 @@ def test_ebe_operator_matches_csr_and_oracle_hex(cuda, tmp_path):
     xs, info = op.solve(b, op.jacobi(), 1e-10, 5000)
     ref = R.ref_pcg([R.CsrPart(sub.A, sub.b)], [1.0 / sub.A.diagonal()], 1e-10, 5000)
     assert info.flag == ref["Flag"] == 0 and abs(info.iters - ref["Iter"]) <= 2
+    # the solution itself: near tol 1e-10 one CG iteration more or less moves x by ~1e-12 relative on this mesh
+    X = ref["X"][0]
+    assert np.linalg.norm(xs.cpu().numpy() - X) <= 1e-10 * np.linalg.norm(X)
 
 
 def test_ebe_operator_concrete(cuda):
